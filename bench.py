@@ -6,7 +6,10 @@ Main workload (configs[1]): SD-XL base 1.0 UNet2DConditionModel, batch 8 per GPU
 denoising timestep = one UNet forward over the batch + the fused DDIM update. Metric = denoiser-forward latents/s
 (images pushed through one denoiser forward per second, whole job); finished latents/s = that / 50.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
+
+K timed steps in every GPU section (SDXL, SD3, STDiT2, Qwen2-VL prefill). --dump-outputs writes what the last timed SDXL
+step returned; inputs and weights are seeded, so runs with the same arguments see identical inputs.
 
 N > 1 is launched by `python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...`: one rank per GPU,
 images sharded, weights replicated, no per-step communication, one NCCL all_gather of the finished latents.
@@ -51,6 +54,7 @@ SD3_TFLOP_PER_SAMPLE = 8.437
 STDIT2_TFLOP_PER_SAMPLE = 24.39
 PARITY_TOL = {"cosine_min": 0.999, "max_rel_err": 0.04}
 REF_STEPS, REF_WARMUP = 3, 1  # reference / cpu_baseline legs: fixed sample count, independent of --steps
+DUMP_BYTES = 64_000_000  # --dump-outputs: upper bound of all files together
 
 
 class ClockSampler(threading.Thread):
@@ -219,6 +223,27 @@ class Ctx:
         return self.max_over_ranks(e0.elapsed_time(e1))[0]
 
 
+def dump_outputs(c, outputs, out_dir):
+    """Writes each device tensor of `outputs` as out_dir/<name>.npy in float32 (rank 0; with N ranks the global batch in
+    rank order). An array over its share of DUMP_BYTES is replaced by a fixed seeded sample of its flattened elements,
+    so two builds run with the same arguments can be compared element for element."""
+    import numpy as np
+    import torch
+    cap = (DUMP_BYTES // len(outputs) - 4096) // 4  # float32 elements per file, .npy header included
+    for name, t in outputs.items():
+        t = t.float().contiguous()
+        if c.world > 1:
+            full = torch.empty((c.world * t.shape[0],) + tuple(t.shape[1:]), device=t.device, dtype=t.dtype)
+            c.dist.all_gather_into_tensor(full, t)
+            t = full
+        if t.numel() > cap:
+            idx = torch.randint(t.numel(), (cap,), generator=torch.Generator().manual_seed(0))
+            t = t.flatten()[idx.to(t.device)]
+        if c.rank == 0:
+            os.makedirs(out_dir, exist_ok=True)
+            np.save(os.path.join(out_dir, f"{name}.npy"), t.cpu().numpy())
+
+
 def sdxl_setup(c, B, height):
     """Model, graph, scheduler and pinned host inputs of the SDXL workload for B images on this rank."""
     import torch
@@ -239,8 +264,9 @@ def sdxl_setup(c, B, height):
     return s
 
 
-def sdxl_section(c, unet, B, height, steps, warmup, with_e2e=True, sample_clocks=False):
-    """Device-resident steps, end-to-end steps (host buffers), job-level (steps + all_gather + D2H) for B images/rank."""
+def sdxl_section(c, unet, B, height, steps, warmup, with_e2e=True, sample_clocks=False, keep_outputs=False):
+    """Device-resident steps, end-to-end steps (host buffers), job-level (steps + all_gather + D2H) for B images/rank.
+    keep_outputs: res["outputs"] holds what the last timed step returned (noise prediction, next latents)."""
     import torch
 
     from paddlemix_b200 import ops
@@ -270,6 +296,8 @@ def sdxl_section(c, unet, B, height, steps, warmup, with_e2e=True, sample_clocks
     if sampler:
         sampler.stop_flag = True
     res = {"ms": ms, "launches": launches, "clocks": sampler.summary() if sampler else None, "den": den, "state": s}
+    if keep_outputs:  # copied now: the job leg below steps the same state further
+        res["outputs"] = {"noise_pred": den.out.float(), "latents": state["lat"].clone()}
 
     # job level: K steps + the path's only collective (all_gather of the finished latents) + D2H of the gathered result
     gathered_h = torch.empty(B * c.world, 4, H, H).pin_memory() if c.rank == 0 else None
@@ -578,7 +606,10 @@ def run_b200(args):
     B, height = args.batch, args.height
     unet = UNet2DConditionModel(**SDXL).init_synthetic_weights(seed=1, device=c.local)
 
-    main = sdxl_section(c, unet, B, height, args.steps, args.warmup, with_e2e=True, sample_clocks=True)
+    main = sdxl_section(c, unet, B, height, args.steps, args.warmup, with_e2e=True, sample_clocks=True,
+                        keep_outputs=args.dump_outputs is not None)
+    if args.dump_outputs is not None:
+        dump_outputs(c, main.pop("outputs"), args.dump_outputs)
     ms, ms_e2e = main["ms"], main["e2e"]["ms"]
     roof = roofline_section(c, unet, B, height) if rank == 0 else None
 
@@ -608,11 +639,11 @@ def run_b200(args):
 
     if not args.no_extras:
         try:
-            extras["sd3_b32"] = sd3_section(c, steps=min(args.steps, 10), warmup=3)
+            extras["sd3_b32"] = sd3_section(c, steps=args.steps, warmup=args.warmup)
         except Exception as ex:  # noqa: BLE001
             extras["sd3_b32"] = {"error": repr(ex)[:300]}
         try:
-            extras["stdit2_b4"] = stdit2_section(c, steps=min(args.steps, 10), warmup=3)
+            extras["stdit2_b4"] = stdit2_section(c, steps=args.steps, warmup=args.warmup)
         except Exception as ex:  # noqa: BLE001
             extras["stdit2_b4"] = {"error": repr(ex)[:300]}
 
@@ -624,7 +655,7 @@ def run_b200(args):
     qwen = None
     if world == 1 and not args.no_qwen:
         try:
-            qwen = bench_qwen2vl_prefill(c.dev)
+            qwen = bench_qwen2vl_prefill(c.dev, steps=args.steps)
         except Exception as ex:  # noqa: BLE001
             qwen = {"metric": "qwen2vl_7b_prefill_tokens_per_sec", "value": None, "error": repr(ex)[:300]}
 
@@ -687,7 +718,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-qwen", action="store_true", help="skip the Qwen2-VL-7B prefill section")
     ap.add_argument("--no-extras", action="store_true", help="skip the strong-scaling / SD3 / STDiT2 sections")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed SDXL steps, write what the last one returned (noise_pred, latents) as "
+                         "float32 DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     if args.impl == "reference":
